@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--scaling weak|strong]   (N>1: torch.distributed.run, one rank / GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W          (the reference's own PyTorch-CPU path)
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR        (also writes the last timed step's mel to DIR)
 
 Headline workload (BASELINE.json configs[1], svc_content_vec.py): the full 100-evaluation DDPM ("naive") sampler of the
 WaveNet denoiser (M=128, E=256, C=512, L=20, dilation cycle 4, timesteps=1000, sampler_interval=10), B=32 items x
@@ -97,6 +98,32 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2], "sm_max_mhz": max(smax), "power_w_max": max(power),
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each [B, T, ...] tensor as out_dir/<name>.npy in float32 so that two builds run with the same arguments can
+    be compared output for output.  A tensor above the byte budget (shared evenly) keeps a sorted, seeded sample of its
+    frames (axis 1), the same for every item and every run.  -> {name: description} for the JSON line."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // len(arrays) - 4096          # room for the .npy header
+    info = {}
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        desc = {"shape": list(a.shape), "dtype": "float32"}
+        if a.nbytes > budget:
+            per_frame = a.nbytes // a.shape[1]
+            frames = np.sort(np.random.default_rng(0).choice(a.shape[1], budget // per_frame, replace=False))
+            a = np.ascontiguousarray(a[:, frames])
+            desc["sample"] = f"{len(frames)} of {desc['shape'][1]} frames (axis 1), np.random.default_rng(0).choice, sorted"
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        desc["file"] = name + ".npy"
+        desc["saved_shape"] = list(a.shape)
+        info[name] = desc
+    return info
 
 
 # ------------------------------------------------------------------------------------------ CPU arm: the reference itself
@@ -273,7 +300,12 @@ def main():
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--no-voc-train", action="store_true", help="skip the vocoder-training side measurement (N4)")
     ap.add_argument("--no-extras", action="store_true", help="skip unipc / single-product / strong-scaling side runs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the mel [B, T, M] that the last timed step returned on rank 0 as "
+                         "DIR/mel.npy (float32; at most 64 MB: a seeded sample of frames when larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -340,10 +372,16 @@ def main():
     clocks = ClockSampler(local)
     clocks.start()
     launches0 = N.launch_count()
-    ms_per_step = timed(sampler_step, args.steps)
+    last = {}
+
+    def timed_step():
+        last["mel"] = sampler_step()
+
+    ms_per_step = timed(timed_step, args.steps)
     launches = N.launch_count() - launches0
     clk = clocks.stop()
     value = global_B * T / (ms_per_step * 1e-3)
+    dumped = dump_outputs(args.dump_outputs, {"mel": last.pop("mel")}) if args.dump_outputs and rank == 0 else None
     # the graph replays launch the same kernels without passing the library's launch counter: count them from one
     # eager evaluation (identical launch sequence) -- kernels per sampler run, all of this repo's own
     diff.denoise_fn.use_graph = False
@@ -528,6 +566,8 @@ def main():
             "kernel_ms": {k: {"total_ms": v[0], "launches": v[1]} for k, v in prof.items()},
         }
         line.update(extras)
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         print(json.dumps(line))
     if world > 1:
         torch.distributed.destroy_process_group()

@@ -10,6 +10,9 @@ discriminators and the losses is the reference's own code (models.py, utils/audi
                  weights = n4_util.fill_discriminators, random draws = RandomState(SEED_DRAWS) in call order),
                  the generator's input mel and output audio, the three logged losses, and norm + 256 sampled entries of
                  every gradient left on the generator and the discriminators after the step.
+  n4_disc.npz    MultiPeriodDiscriminator([3, 5]) and MultiScaleDiscriminator() of the reference in train mode: state_dict
+                 names and shapes, the logits, norm + 256 sampled entries of every feature map, and the three losses on
+                 n4_util.disc_inputs() with n4_util.fill_discriminators weights.
 """
 import json
 import os
@@ -155,6 +158,49 @@ def main():
     # the checkpoint holds 3x the reference's initial weights (round-2 golden: audible output), which saturates the final
     # tanh (rms 0.9998); a third of it is the reference's own initialisation -- a well-conditioned operating point
     gold_generator_grads(ref, {k: v / 3 for k, v in sd.items()}, out["mels"], out["pitches"], 1.0 / 3, "n4_gen_init.npz")
+    gold_discriminators(ref)
+
+
+def gold_discriminators(ref):
+    """n4_disc.npz: the reference discriminators' forward in float32 (8 threads).  oneDNN's grouped convolutions of the
+    multi-scale discriminator round differently with the thread count, so the same module on the same CPU moves in the
+    last bits; the largest such move over 1, 3 and 8 threads is stored as `noise_<tag>`."""
+    out = {}
+    y, yh = (torch.from_numpy(a) for a in nu.disc_inputs())
+    for tag, make in (("mpd", lambda: ref.nsf.MultiPeriodDiscriminator([3, 5])), ("msd", ref.nsf.MultiScaleDiscriminator)):
+        runs = {}
+        for nt in (1, 3, 8):
+            torch.set_num_threads(nt)
+            m = make()
+            nu.fill_discriminators(m)
+            m.train()
+            with torch.no_grad():
+                runs[nt] = m(y, yh)
+        sd = m.state_dict()
+        out[f"{tag}_keys"] = np.array(list(sd))
+        out[f"{tag}_shapes"] = np.array([list(v.shape) + [0] * (4 - v.dim()) for v in sd.values()], dtype=np.int64)
+        d_r, d_g, f_r, f_g = runs[8]
+        noise = 0.0
+        for side, logits, fmaps in (("r", d_r, f_r), ("g", d_g, f_g)):
+            for i, t in enumerate(logits):
+                out[f"{tag}_logit_{side}{i}"] = t.numpy()
+                for nt in (1, 3):
+                    o = runs[nt][0 if side == "r" else 1][i]
+                    noise = max(noise, float((o - t).norm() / t.norm()))
+            for i, maps in enumerate(fmaps):
+                for j, t in enumerate(maps):
+                    nu.summarize(out, f"{tag}_fmap_{side}{i}_{j}", t.numpy(), 4600 + 10 * i + j)
+                    for nt in (1, 3):
+                        o = runs[nt][2 if side == "r" else 3][i][j]
+                        noise = max(noise, float((o - t).norm() / t.norm()))
+        out[f"noise_{tag}"] = np.float64(noise)
+        out[f"{tag}_feature_loss"] = np.float64(float(ref.nsf.feature_loss(f_r, f_g)))
+        out[f"{tag}_discriminator_loss"] = np.float64(float(ref.nsf.discriminator_loss(d_r, d_g)[0]))
+        out[f"{tag}_generator_loss"] = np.float64(float(ref.nsf.generator_loss(d_g)[0]))
+        print(f"  {tag}: thread-count noise {noise:.2e}")
+    torch.set_num_threads(8)
+    np.savez_compressed(os.path.join(HERE, "n4_disc.npz"), **out)
+    print("n4_disc.npz:", os.path.getsize(os.path.join(HERE, "n4_disc.npz")) // 1024, "KiB")
 
 
 def gold_generator_grads(ref, sd, mels, pitches, scale, fname):

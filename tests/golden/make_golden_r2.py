@@ -16,6 +16,7 @@ and the recorded-random machinery).  Run in the build container:  python tests/g
                      the executed code path touches neither.
   r2_diffsinger.npz  archs/diffsinger/diffsinger.py DiffSinger.forward_features / forward (+ NaiveProjectionEncoder,
                      pitch_to_scale) with the un-importable Lightning-side names stubbed: features, masks, loss, encoder grads.
+  r2_warmup_cosine.npz  schedulers/warmup_cosine_scheduler.py: the learning-rate multiplier over a set of steps.
   ref_ckpt_small.ckpt / ref_generator_small.ckpt   checkpoints WRITTEN by the reference classes (state_dict of the
                      reference GaussianDiffusion under Lightning's `model.diffusion.` prefix with an `ema_model.` copy; the
                      reference Generator with weight-norm keys as {"generator": ...}) plus the reference outputs.
@@ -341,12 +342,29 @@ def gold_diffsinger(ref, out):
     print(f"  diffsinger: features {tuple(f['features'].shape)}, loss {float(o['loss']):.5f}, draws {[k for k, _ in rr.log]}")
 
 
+def gold_warmup_cosine(ref, out):
+    """schedulers/warmup_cosine_scheduler.py LambdaWarmUpCosineScheduler with the warmup_cosine config's values: the
+    multiplier and `last_lr` after each call, at every 7th step of the warm-up and around its ends."""
+    sch = mg._load("ref_warmup_cosine", f"{REF}/fish_diffusion/schedulers/warmup_cosine_scheduler.py")
+    out["kwargs"] = np.array(json.dumps(dict(warm_up_steps=1000, val_final=2e-5, val_base=8e-4, val_start=1e-5,
+                                             max_decay_steps=300000)))
+    s = sch.LambdaWarmUpCosineScheduler(**json.loads(str(out["kwargs"])))
+    steps = list(range(0, 1200, 7)) + [999, 1000, 1001, 5000, 123456, 299999, 300000, 300001, 2_000_000]
+    out["steps"] = np.array(steps, dtype=np.int64)
+    vals, last = [], []
+    for n in steps:
+        vals.append(s(n))
+        last.append(s.last_lr)
+    out["lr"], out["last_lr"] = np.array(vals, dtype=np.float64), np.array(last, dtype=np.float64)
+
+
 def main():
     torch.manual_seed(0)
     torch.set_num_threads(8)
     ref = mg.load_reference()
     groups = {"traj": gold_traj, "train_full": gold_train_full, "train_masked": gold_train_masked, "voc": gold_voc,
-              "audio": gold_audio, "ckpt": gold_ckpt, "diffsinger": gold_diffsinger, "voc_resblock2": gold_voc_resblock2}
+              "audio": gold_audio, "ckpt": gold_ckpt, "diffsinger": gold_diffsinger, "voc_resblock2": gold_voc_resblock2,
+              "warmup_cosine": gold_warmup_cosine}
     only = sys.argv[1:]
     for name, fn in groups.items():
         if only and name not in only:

@@ -65,6 +65,12 @@ def make_batch():
                 audio_lens=torch.tensor([S, S - 3 * hop], dtype=torch.long))
 
 
+def disc_inputs():
+    """-> (y, y_hat) [2, 1, 2050] float32: real and generated audio for the discriminator comparison."""
+    rng = np.random.RandomState(4250)
+    return rng.randn(2, 1, 2050).astype(np.float32), rng.randn(2, 1, 2050).astype(np.float32)
+
+
 def summarize(out, key, arr, seed, samples=256):
     a = np.asarray(arr, dtype=np.float32).reshape(-1)
     idx = np.random.RandomState(seed).randint(0, a.size, size=min(samples, a.size))

@@ -216,20 +216,24 @@ def test_reference_written_checkpoint_loads_strictly(golden_cfg):
 
 
 def test_oracle_ref_copy_is_verbatim():
-    """oracle/_ref (the files the CPU baseline runs) are byte-identical to /root/reference when both are present."""
+    """oracle/_ref (the files the CPU baseline runs, copied by build() where the reference is installed) is byte-identical
+    to the reference release the golden vectors were made from (tests/golden/ref_sha256.json)."""
     import hashlib
     import json as _json
     import os
+    from conftest import GOLDEN
     from oracle.ref_loader import REF_FILES
     here = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
-    if not (os.path.isdir(here) and os.path.isdir("/root/reference")):
-        pytest.skip("needs both /root/reference and oracle/_ref")
-    man = _json.load(open(os.path.join(here, "MANIFEST.json")))["sha256"]
+    if not os.path.isdir(here):
+        pytest.skip("oracle/_ref not built: the reference is not installed on this machine")
+    with open(os.path.join(GOLDEN, "ref_sha256.json")) as f:
+        want = _json.load(f)
+    with open(os.path.join(here, "MANIFEST.json")) as f:
+        man = _json.load(f)["sha256"]
     for rel in REF_FILES:
-        with open(os.path.join("/root/reference", rel), "rb") as f:
-            assert hashlib.sha256(f.read()).hexdigest() == man[rel], rel
+        assert man[rel] == want[rel], rel
         with open(os.path.join(here, rel), "rb") as f:
-            assert hashlib.sha256(f.read()).hexdigest() == man[rel], rel
+            assert hashlib.sha256(f.read()).hexdigest() == want[rel], rel
 
 
 def test_step_vectors_batched_projection_matches_per_layer_definition():
