@@ -20,7 +20,7 @@ PREC_F16, PREC_BF16 = 0, 1
 PREC_SINGLE = 0x10   # or-ed into the prec of GEMM calls: one product over the hi planes
 BACKEND_TC, BACKEND_SIMT = 0, 1
 ACT_NONE, ACT_RELU, ACT_LRELU = 0, 1, 2
-ABI_VERSION = 1
+ABI_VERSION = 2
 
 
 class NativeError(RuntimeError):
@@ -70,7 +70,8 @@ class ResPairDesc(ctypes.Structure):
 class WaveNetFwdDesc(ctypes.Structure):
     """struct fd_wavenet_fwd_desc (include/fishdiff_b200.h)."""
     _fields_ = [
-        ("x_planes", c_void_p), ("cond_planes", c_void_p), ("steps", c_void_p), ("x_mask", c_void_p), ("out", c_void_p),
+        ("x_planes", c_void_p), ("cond_planes", c_void_p), ("cond_term", c_void_p), ("steps", c_void_p),
+        ("x_mask", c_void_p), ("out", c_void_p),
         ("w_in", c_void_p), ("b_in", c_void_p), ("w_in_inv", c_float),
         ("mlp_w0", c_void_p), ("mlp_b0", c_void_p), ("mlp_w1", c_void_p), ("mlp_b1", c_void_p),
         ("wd", c_void_p), ("bd", c_void_p), ("w1p_f32", c_void_p), ("bias_sum", c_void_p),
@@ -145,6 +146,8 @@ _SIGS = {
     "fd_wavenet_block_fwd": (c_int, [c_void_p] * 8 + [c_int, c_void_p, c_void_p, c_void_p, c_float] + [c_int] * 6 +
                              [c_float, c_float, c_int, c_int, c_int, c_void_p]),
     "fd_wavenet_fwd": (c_int, [POINTER(WaveNetFwdDesc), c_void_p]),
+    "fd_wavenet_cond_term": (c_int, [c_void_p, c_void_p, c_longlong, POINTER(c_float), c_void_p] + [c_int] * 7 +
+                             [c_void_p]),
     "fd_conv_cl_fwd": (c_int, [POINTER(ConvDesc), c_void_p]),
     "fd_respair_supported": (c_int, [c_int, c_int, c_int, c_int]),
     "fd_respair_fwd": (c_int, [POINTER(ResPairDesc), c_void_p]),

@@ -140,7 +140,7 @@ int fd_tc_supported_linear(int n_total, int k_seg, int num_seg) {
 }
 
 static int wavenet_block(const uint16_t* x_planes, uint16_t* x_out_planes, const uint16_t* cond_planes,
-                         uint16_t* z_planes, uint16_t* y_planes, const uint16_t* w1, const uint16_t* w2,
+                         const float* cond_term, uint16_t* z_planes, uint16_t* y_planes, const uint16_t* w1, const uint16_t* w2,
                          const float* gb_full, const float* gb_lo, const float* gb_hi, int gb_bstride, const float* b2,
                          float* skip_f32, uint16_t* skip_planes, float skip_scale, int B, int T, int C, int E,
                          int dilation, int gate_tile, float w1_inv_scale, float w2_inv_scale, int flags, int prec,
@@ -152,7 +152,7 @@ int fd_wavenet_block_fwd(uint16_t* x_planes, const uint16_t* cond_planes, uint16
                          int B, int T, int C, int E, int dilation, int gate_tile, float w1_inv_scale,
                          float w2_inv_scale, int flags, int prec, int backend, void* stream) {
   FD_DEVICE_GUARD();
-  return wavenet_block(x_planes, nullptr, cond_planes, z_planes, nullptr, w1, w2, gb_full, gb_lo, gb_hi, gb_bstride, b2,
+  return wavenet_block(x_planes, nullptr, cond_planes, nullptr, z_planes, nullptr, w1, w2, gb_full, gb_lo, gb_hi, gb_bstride, b2,
                        skip_f32, skip_planes, skip_scale, B, T, C, E, dilation, gate_tile, w1_inv_scale, w2_inv_scale,
                        flags, prec, backend, stream);
 }
@@ -165,13 +165,13 @@ int fd_wavenet_block_fwd_train(const uint16_t* x_planes, uint16_t* x_out_planes,
                                int flags, int prec, int backend, void* stream) {
   FD_DEVICE_GUARD();
   FD_REQUIRE(x_out_planes != nullptr && y_planes != nullptr, "fd_wavenet_block_fwd_train: x_out / y planes required");
-  return wavenet_block(x_planes, x_out_planes, cond_planes, z_planes, y_planes, w1, w2, gb_full, gb_lo, gb_hi,
+  return wavenet_block(x_planes, x_out_planes, cond_planes, nullptr, z_planes, y_planes, w1, w2, gb_full, gb_lo, gb_hi,
                        gb_bstride, b2, skip_f32, skip_planes, skip_scale, B, T, C, E, dilation, gate_tile, w1_inv_scale,
                        w2_inv_scale, flags, prec, backend, stream);
 }
 
 static int wavenet_block(const uint16_t* x_planes, uint16_t* x_out_planes, const uint16_t* cond_planes,
-                         uint16_t* z_planes, uint16_t* y_planes, const uint16_t* w1, const uint16_t* w2,
+                         const float* cond_term, uint16_t* z_planes, uint16_t* y_planes, const uint16_t* w1, const uint16_t* w2,
                          const float* gb_full, const float* gb_lo, const float* gb_hi, int gb_bstride, const float* b2,
                          float* skip_f32, uint16_t* skip_planes, float skip_scale, int B, int T, int C, int E,
                          int dilation, int gate_tile, float w1_inv_scale, float w2_inv_scale, int flags, int prec,
@@ -179,17 +179,20 @@ static int wavenet_block(const uint16_t* x_planes, uint16_t* x_out_planes, const
   FD_REQUIRE(B > 0 && T > 0 && C > 0 && E > 0 && dilation > 0, "fd_wavenet_block_fwd: bad shape");
   FD_REQUIRE(C % 8 == 0 && E % 8 == 0, "fd_wavenet_block_fwd: C=%d, E=%d must be multiples of 8", C, E);
   cudaStream_t st = (cudaStream_t)stream;
-  // ---- GEMM1: dilated conv (3 taps) + conditioner projection + gate
+  // ---- GEMM1: dilated conv (3 taps) + conditioner projection + gate.  With cond_term (W_cond . cond computed once per
+  //      sampler call, fd_wavenet_cond_term) the launch reads only the tap columns [0, 3C) of the packed W1 and adds the
+  //      conditioner term in the epilogue.
   FdTapGemm p;
   init_desc(p);
   p.B = B; p.T = T; set_prec(p, prec);
-  p.n_total = 2 * C; p.k_total = 3 * C + E; p.num_seg = 4;
+  p.n_total = 2 * C; p.k_total = 3 * C + E; p.num_seg = cond_term != nullptr ? 3 : 4;
   p.seg[0] = FdSeg{0, -dilation, 0, C};
   p.seg[1] = FdSeg{0, 0, 0, C};
   p.seg[2] = FdSeg{0, dilation, 0, C};
   p.seg[3] = FdSeg{1, 0, 0, E};
   set_src(p, 0, x_planes, C);
-  set_src(p, 1, cond_planes, E);
+  if (cond_term != nullptr) p.addend = cond_term;
+  else set_src(p, 1, cond_planes, E);
   p.w = w1; p.acc_scale = w1_inv_scale;
   p.epi = FD_EPI_GATE;
   p.gbias_full = gb_full; p.gbias_lo = gb_lo; p.gbias_hi = gb_hi; p.gbias_bstride = gb_bstride;
@@ -241,11 +244,11 @@ int fd_wavenet_fwd(const fd_wavenet_fwd_desc* d, void* stream) {
   for (int l = 0; l < L; ++l) {
     const int flags = (l == 0 ? 1 : 0) | (l == L - 1 ? 2 : 0);
     const size_t go = (size_t)l * Bs * 2 * C;
-    rc = fd_wavenet_block_fwd(d->xr, d->cond_planes, d->z, d->w1 + (size_t)l * d->w1_lstride,
-                              d->w2 + (size_t)l * d->w2_lstride, gb_full + go, gb_lo + go, gb_hi + go, gb_stride,
-                              d->b2 + (size_t)l * d->b2_lstride, d->skip_f32, d->skip_planes, skip_scale, B, T, C, E,
-                              d->dilation[l], d->gate_tile, d->w1_inv[l], d->w2_inv[l], flags, d->prec, d->backend,
-                              stream);
+    const float* ct = d->cond_term != nullptr ? d->cond_term + (size_t)l * B * T * 2 * C : nullptr;
+    rc = wavenet_block(d->xr, nullptr, d->cond_planes, ct, d->z, nullptr, d->w1 + (size_t)l * d->w1_lstride,
+                       d->w2 + (size_t)l * d->w2_lstride, gb_full + go, gb_lo + go, gb_hi + go, gb_stride,
+                       d->b2 + (size_t)l * d->b2_lstride, d->skip_f32, d->skip_planes, skip_scale, B, T, C, E,
+                       d->dilation[l], d->gate_tile, d->w1_inv[l], d->w2_inv[l], flags, d->prec, d->backend, stream);
     if (rc) return rc;
   }
   // tail: relu(skip_projection(sum / sqrt(L))) -> output_projection, masked rows zeroed (wavenet.py:228-234)
@@ -256,6 +259,29 @@ int fd_wavenet_fwd(const fd_wavenet_fwd_desc* d, void* stream) {
   cd.in_planes = d->z; cd.w_planes = d->w_out; cd.bias = d->b_out; cd.row_mask = d->x_mask;
   cd.out_planes = nullptr; cd.out_f32 = d->out; cd.Cin = C; cd.N = M; cd.w_inv_scale = d->w_out_inv; cd.act = 0;
   return fd_conv_cl_fwd(&cd, stream);
+}
+
+int fd_wavenet_cond_term(const uint16_t* cond_planes, const uint16_t* w1, long long w1_lstride, const float* w1_inv,
+                         float* cond_term, int L, int B, int T, int C, int E, int prec, int backend, void* stream) {
+  FD_DEVICE_GUARD();
+  FD_REQUIRE(L >= 1 && L <= 64, "fd_wavenet_cond_term: L=%d out of range (1..64)", L);
+  FD_REQUIRE(B > 0 && T > 0 && C > 0 && E > 0, "fd_wavenet_cond_term: bad shape");
+  FD_REQUIRE(C % 8 == 0 && E % 8 == 0, "fd_wavenet_cond_term: C=%d, E=%d must be multiples of 8", C, E);
+  for (int l = 0; l < L; ++l) {
+    FdTapGemm p;
+    init_desc(p);
+    p.B = B; p.T = T; set_prec(p, prec);
+    p.n_total = 2 * C; p.k_total = 3 * C + E; p.num_seg = 1;
+    p.seg[0] = FdSeg{0, 0, 0, E};
+    set_src(p, 0, cond_planes, E);
+    p.w = w1 + (size_t)l * w1_lstride; p.w_kshift = 3 * C;   // the conditioner columns of the packed W1
+    p.acc_scale = w1_inv[l];
+    p.epi = FD_EPI_LINEAR;
+    p.out_f32 = cond_term + (size_t)l * B * T * 2 * C;
+    const int rc = run(p, backend, (cudaStream_t)stream);
+    if (rc) return rc;
+  }
+  return 0;
 }
 
 int fd_conv_cl_fwd(const fd_conv_desc* d, void* stream) {

@@ -43,7 +43,7 @@ struct FdTapGemm {
   // ---- problem: D[b,t,n] = sum_seg sum_k src[seg.src][b, t+seg.shift, seg.c_off+k] * W[n, koff(seg)+k]
   int B, T;
   int n_total;   // output columns (rows of W)
-  int k_total;   // sum of seg.k_len (row pitch of W)
+  int k_total;   // row pitch of W: sum of seg.k_len, or more when the launch reads only the leading columns
   int num_seg;
   int prec;      // FD_F16 / FD_BF16
   int single;    // 1: one product over the hi planes (half-precision operands), 0: three split products
@@ -82,8 +82,10 @@ struct FdTapGemm {
 
   // ---- FD_EPI_GATE (WaveNet GEMM1): column tile of width NT holds NT/2 gate columns followed by
   //      NT/2 filter columns for residual channels [tile*NT/2, (tile+1)*NT/2).
-  //      y = acc*acc_scale + gbias_full[n] - (t<dil ? gbias_lo[n] : 0) - (t+dil>=T ? gbias_hi[n] : 0)
+  //      y = acc*acc_scale + gbias_full[n] - (t<dil ? gbias_lo[n] : 0) - (t+dil>=T ? gbias_hi[n] : 0) + addend[b,t,n]
   //      z = sigmoid(y_gate) * tanh(y_filter)  -> out_planes [2][B][T][C]
+  //      addend (fp32 [B][T][n_total] in packed column order, or null) carries the conditioner projection when the
+  //      sampler computed it once per call instead of as a K segment of every evaluation
   const float* gbias_full;  // [Bs][n_total]  (conv bias + cond bias + sum over 3 taps of W_tap.d)
   const float* gbias_lo;    // [Bs][n_total]  tap-0 (t-dil) contribution of the step vector
   const float* gbias_hi;    // [Bs][n_total]  tap-2 (t+dil) contribution
@@ -354,13 +356,21 @@ __device__ __forceinline__ void fd_epi_gate(const FdTapGemm& p, int b, int t, in
     if (e_lo) { yg -= lo_g[i]; yf -= lo_f[i]; }
     if (e_hi) { yg -= hi_g[i]; yf -= hi_f[i]; }
     yg8[i] = yg; yf8[i] = yf;
-    z[i] = fd_sigmoid(yg) * fd_tanh(yf);
   }
+  const int half = p.gate_tile / 2;
+  const int ng = (zc0 / half) * p.gate_tile + (zc0 % half);   // packed column of the first gate channel
+  const size_t yoff = ((size_t)b * p.T + t) * p.n_total;
+  if (p.addend != nullptr) {
+    float ag[V], af[V];
+    fd_load_f32<V>(p.addend + yoff + ng, ag);
+    fd_load_f32<V>(p.addend + yoff + ng + half, af);
+#pragma unroll
+    for (int i = 0; i < V; ++i) { yg8[i] += ag[i]; yf8[i] += af[i]; }
+  }
+#pragma unroll
+  for (int i = 0; i < V; ++i) z[i] = fd_sigmoid(yg8[i]) * fd_tanh(yf8[i]);
   if (p.y_planes != nullptr) {   // training: keep the pre-activations (packed column order: gates | filters per tile)
-    const int half = p.gate_tile / 2;
-    const int ng = (zc0 / half) * p.gate_tile + (zc0 % half);
     const size_t yplane = (size_t)p.B * p.T * p.n_total;
-    const size_t yoff = ((size_t)b * p.T + t) * p.n_total;
     fd_store_planes<V>(p.y_planes, yplane, yoff + ng, yg8, prec);
     fd_store_planes<V>(p.y_planes, yplane, yoff + ng + half, yf8, prec);
   }

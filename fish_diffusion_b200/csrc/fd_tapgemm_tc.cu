@@ -259,9 +259,21 @@ fd_tapgemm_tc_kernel(const __grid_constant__ CUtensorMap tm_src0, const __grid_c
         const size_t zplane = (size_t)p.B * p.T * p.C, zrow = ((size_t)b * p.T + t) * p.C + (size_t)n_tile * HALF;
         const size_t yplane = (size_t)p.B * p.T * p.n_total, yrow = ((size_t)b * p.T + t) * p.n_total;
         const int halfg = p.gate_tile / 2;
+        // conditioner term of the hoisted sampler path (fp32, packed column order like the accumulator tile)
+        const bool has_add = EPI == FD_EPI_GATE && p.addend != nullptr && valid;
+        const float* const add_row = has_add ? p.addend + yrow + n0 : nullptr;
         for (int c = 0; c < PER; c += 16) {
           const int c0 = cb + c;
           float g[16], f[16];
+          // this row's 2 x 64 bytes of the addend are requested before the TMEM wait, so their latency overlaps it
+          float4 ag[4], af[4];
+          if (has_add) {
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+              ag[i] = __ldg(reinterpret_cast<const float4*>(add_row + c0) + i);
+              af[i] = __ldg(reinterpret_cast<const float4*>(add_row + HALF + c0) + i);
+            }
+          }
           tmem_ld16_nowait(taddr + c0, g);
           tmem_ld16_nowait(taddr + HALF + c0, f);
           tmem_wait16(g);
@@ -301,6 +313,13 @@ fd_tapgemm_tc_kernel(const __grid_constant__ CUtensorMap tm_src0, const __grid_c
                       for (int i = 0; i < 8; ++i) { yg[i] -= eg[i]; yf[i] -= ef[i]; }
                     }
                   }
+                }
+                if (has_add) {
+                  const float4 a0 = ag[2 * h], a1 = ag[2 * h + 1], b0 = af[2 * h], b1 = af[2 * h + 1];
+                  const float eg[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+                  const float ef[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+#pragma unroll
+                  for (int i = 0; i < 8; ++i) { yg[i] += eg[i]; yf[i] += ef[i]; }
                 }
 #pragma unroll
                 for (int i = 0; i < 8; ++i) z[i] = fd_sigmoid(yg[i]) * fd_tanh(yf[i]);

@@ -10,6 +10,7 @@ Scalar coefficient math stays on the host exactly like the reference's float32 b
 from __future__ import annotations
 
 import json
+import math
 from functools import partial
 
 import numpy as np
@@ -19,6 +20,10 @@ from torch import nn
 from . import _native as N
 from .registry import DENOISERS, DIFFUSIONS
 from .uni_pc import NoiseScheduleVP, unipc_sample_native
+
+# Largest per-call buffer of hoisted conditioner projections (fp32 [L, B, T, 2C]; 10.5 GB at L=20, C=512, B=32, T=4000)
+# the sampler keeps; a call that would need more multiplies the conditioner inside every evaluation instead.
+COND_TERM_BUDGET_BYTES = 16 << 30
 
 
 def get_noise_schedule_list(schedule_mode, timesteps, max_beta=0.01, s=0.008):
@@ -357,6 +362,14 @@ class GaussianDiffusion(nn.Module):
         elif cond_planes.data_ptr() != ws["cond_planes"].data_ptr():
             ws["cond_planes"].copy_(cond_planes)
             cond_planes = ws["cond_planes"]
+        # the conditioner projections of every layer are computed once per call here instead of inside each
+        # evaluation's gate GEMM (a seventh of its multiply work); above the byte budget the evaluations keep doing it
+        cond_term = None
+        ct_shape = (den.n_layers, B, T, 2 * den.residual_channels)
+        if math.prod(ct_shape) * 4 <= COND_TERM_BUDGET_BYTES:
+            if ws.get("cond_term") is None or tuple(ws["cond_term"].shape) != ct_shape:
+                ws["cond_term"] = torch.empty(ct_shape, dtype=torch.float32, device=dev)
+            cond_term = den.cond_term(cond_planes, out=ws["cond_term"])
         if original_mel is None:
             x = self._to_cl(x_T) if x_T is not None else self._randn((B, T, M), dev, out=ws["x"])
         else:
@@ -391,7 +404,8 @@ class GaussianDiffusion(nn.Module):
             steps = step_table.get(t_float)
             if steps is None:
                 steps = step_table[t_float] = torch.tensor([t_float], dtype=torch.float32, device=dev)
-            return den.forward_cl(xp, steps, cond_planes, x_mask=x_masks if masks else None, out=out)
+            return den.forward_cl(xp, steps, cond_planes, x_mask=x_masks if masks else None, out=out,
+                                  cond_term=cond_term)
 
         if noise_predictor in ("naive", "plms") and len(chunks) > 1:   # one upload for the whole schedule
             tab = torch.tensor([float(t) for t in chunks], dtype=torch.float32, device=dev)

@@ -332,11 +332,29 @@ class WaveNet(nn.Module):
 
     # ------------------------------------------------------------------------------------ native forward
     @torch.no_grad()
-    def forward_cl(self, x_planes, steps, cond_planes, x_mask=None, out=None):
+    def cond_term(self, cond_planes, out):
+        """W_cond . cond of every residual layer (fd_wavenet_cond_term) -> out fp32 [L,B,T,2C] (packed gate/filter column
+        order, no bias).  cond is the same for every evaluation of a sampler call, so the sampler computes this once and
+        hands it to forward_cl(cond_term=...), whose gate GEMMs then multiply only the three conv taps."""
+        dev = cond_planes.device
+        N.require_cuda(cond_planes, "cond_planes")
+        _, B, T, E = cond_planes.shape
+        C, L = self.residual_channels, self.n_layers
+        assert E == self.d_encoder and tuple(out.shape) == (L, B, T, 2 * C) and out.dtype == torch.float32
+        pk = self._packed(dev)
+        w1s = self._pack_static["w1"]
+        w1_inv = (ctypes.c_float * L)(*pk["w1_inv"])
+        N.check(N.lib().fd_wavenet_cond_term(N.ptr(cond_planes), N.ptr(w1s), w1s.stride(0), w1_inv, N.ptr(out), L, B, T,
+                                             C, E, pk["mma"], pk["backend"], N.stream_ptr(dev)), "fd_wavenet_cond_term")
+        return out
+
+    @torch.no_grad()
+    def forward_cl(self, x_planes, steps, cond_planes, x_mask=None, out=None, cond_term=None):
         """Channels-last entry used by the fused sampler.
 
         x_planes [2,B,T,M] int16 split planes, steps float32 [1] or [B] (device), cond_planes [2,B,T,E],
-        x_mask uint8/bool [B,T] or None (True = masked).  Returns eps fp32 [B,T,M]."""
+        x_mask uint8/bool [B,T] or None (True = masked), cond_term: None or cond_term(cond_planes) computed with the
+        current weights.  Returns eps fp32 [B,T,M]."""
         dev = x_planes.device
         N.require_cuda(x_planes, "x_planes")
         _, B, T, M = x_planes.shape
@@ -361,18 +379,21 @@ class WaveNet(nn.Module):
         # which also removes the per-launch tensor-map encodes from the host path.
         steps_buf = ws["steps"]
         steps_buf.copy_(steps, non_blocking=True)
+        if cond_term is not None:
+            assert tuple(cond_term.shape) == (L, B, T, 2 * C) and cond_term.dtype == torch.float32
         d = self._fwd_desc(pk, ws, x_planes, cond_planes, steps_buf, x_mask, out, B, T, Bs)
+        d.cond_term = N.ptr(cond_term)
         use_graph = self.use_graph and not N.prof_is_on()
         if not use_graph:
             N.check(lib.fd_wavenet_fwd(ctypes.byref(d), st), "fd_wavenet_fwd")
             return out
-        key = (x_planes.data_ptr(), cond_planes.data_ptr(), out.data_ptr(), 0 if x_mask is None else x_mask.data_ptr(),
-               B, T, Bs, self._pack_key, id(ws))
+        key = (x_planes.data_ptr(), cond_planes.data_ptr(), 0 if cond_term is None else cond_term.data_ptr(),
+               out.data_ptr(), 0 if x_mask is None else x_mask.data_ptr(), B, T, Bs, self._pack_key, id(ws))
         ent = self._graphs.get(key)
         if ent is None:                      # first sight of these buffers: run eagerly (lazy inits happen here)
             if len(self._graphs) >= 4:
                 self._graphs.clear()
-            self._graphs[key] = {"graph": None, "keep": (x_planes, cond_planes, out, x_mask, pk)}
+            self._graphs[key] = {"graph": None, "keep": (x_planes, cond_planes, cond_term, out, x_mask, pk)}
             N.check(lib.fd_wavenet_fwd(ctypes.byref(d), st), "fd_wavenet_fwd")
             return out
         if ent["graph"] is None:

@@ -32,7 +32,7 @@ extern "C" {
 #define FD_PREC_SINGLE 0x10
 #define FD_BACKEND_TC 0
 #define FD_BACKEND_SIMT 1
-#define FD_ABI_VERSION 1
+#define FD_ABI_VERSION 2
 
 /* ------------------------------------------------------------------------------------------- misc */
 int fd_abi_version(void);
@@ -105,6 +105,8 @@ int fd_wavenet_gate_bias(const float* s, const float* wd, const float* bd, const
 typedef struct fd_wavenet_fwd_desc {
   const uint16_t* x_planes;     /* [2][B][T][M] */
   const uint16_t* cond_planes;  /* [2][B][T][E] */
+  const float* cond_term;       /* NULL, or the conditioner projections of fd_wavenet_cond_term [L][B][T][2C]: each GEMM1
+                                   then multiplies only the three conv taps (K = 3C) and adds its layer's slice */
   const float* steps;           /* [Bs] diffusion steps (float), Bs = 1 or B */
   const uint8_t* x_mask;        /* [B][T] or NULL (wavenet.py:217-218, 233-234) */
   float* out;                   /* eps fp32 [B][T][M] */
@@ -126,6 +128,14 @@ typedef struct fd_wavenet_fwd_desc {
   int gate_tile, prec, backend;
 } fd_wavenet_fwd_desc;
 int fd_wavenet_fwd(const fd_wavenet_fwd_desc* d, void* stream);
+
+/* Conditioner projection of every residual layer, computed once for all evaluations of a sampler call (cond does not
+ * change between them):  cond_term[l][b][t][n] = sum_e W1[l][n][3C + e] * cond[b][t][e] * w1_inv[l]  (fp32, the packed
+ * gate/filter column order of w1, no bias: the conditioner bias is part of the gate-bias table).  One linear tap-GEMM
+ * per layer over the conditioner columns of the same packed w1 [L][2][2C][3C+E] that fd_wavenet_fwd reads.
+ * w1_inv: host array [L].  Rows that were zeroed in cond_planes give zeros. */
+int fd_wavenet_cond_term(const uint16_t* cond_planes, const uint16_t* w1, long long w1_lstride, const float* w1_inv,
+                         float* cond_term, int L, int B, int T, int C, int E, int prec, int backend, void* stream);
 
 /* One ResidualBlock.forward (wavenet.py:106-120), fused as two tap-GEMM launches:
  *   GEMM1  y = [W_conv(3 taps) | W_cond] . [x(t-d), x(t), x(t+d), cond(t)] + gate bias ; z = sigmoid(y_g)*tanh(y_f)
